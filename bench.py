@@ -2,9 +2,9 @@
 """bench.py -- BASELINE.json's metric on B200s: SAE training tokens/sec + run_with_cache images/sec, % of roofline.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload all|sae|vit]
-                    [--dtype fp32|bf16] [--batch B] [--model b32|l14]
+                    [--dtype fp32|bf16] [--batch B] [--model b32|l14] [--dump-outputs DIR]
 
-The default invocation (what the driver runs) measures BOTH hot paths and prints ONE JSON line:
+The default invocation measures BOTH hot paths and prints ONE JSON line:
 
   top level    the SAE training step (cfg #3: d_model 768, dict 768 x 32, TopK k = 32, 4096 tokens per step per GPU, fp32) driven
                through the public ``VisionSAETrainer.train_step`` -- the first half of BASELINE.json's metric and the only path with
@@ -23,7 +23,9 @@ Per record:
   dp_parity  (N > 1) after the timed region every rank re-trains the reference-made fixture tests/golden/sae_tiny_b.pt through
              ``VisionSAETrainer(p2p_group=...)`` and compares losses, TopK indices, parameters and counters with the
              single-process reference run; a mismatch makes the process exit non-zero.
-``--impl reference`` times the CPU implementation (the oracle port; /root/reference does not exist on the GPU box).
+``--impl reference`` times the CPU implementation (the oracle port of the reference).
+``--dump-outputs DIR`` writes what every timed path returned to its caller in its last timed step as DIR/<record>.<name>.npy
+(OutputDump); the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -41,6 +43,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "vit-prisma_b200"))
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 SAE_CFG = dict(d_in=768, expansion=32, k=32, batch=4096, dtype="float32")     # BASELINE.json configs[2]
@@ -186,6 +189,34 @@ class Ctx:
         return float(t.item())
 
 
+class OutputDump:
+    """``--dump-outputs DIR``: the arrays a timed path handed its caller in its last timed step, written as DIR/<name>.npy in
+    float32 (floating point) or float64 (integers, exact).  ``add`` copies to the host at once: the next call of the same path
+    rewrites the engine's and the model's output buffers in place.  An array of more than ``cap`` elements is reduced to ``cap``
+    flattened entries at positions drawn from a fixed seed (the same positions in every run), so the files stay under BUDGET."""
+    BUDGET = 64 << 20
+
+    def __init__(self, root):
+        self.root, self.arrays = root, {}
+
+    def add(self, name, value, cap=1 << 20):
+        if value is None:
+            return
+        t = torch.as_tensor(value).detach()
+        if t.numel() > cap:
+            pos = torch.randint(t.numel(), (cap,), generator=torch.Generator().manual_seed(0))
+            t = t.reshape(-1)[pos.to(t.device)]
+        self.arrays[name] = t.to("cpu", torch.float32 if t.is_floating_point() else torch.float64).numpy()
+
+    def write(self):
+        total = sum(a.nbytes for a in self.arrays.values())
+        if total > self.BUDGET:
+            raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes, more than {self.BUDGET}")
+        os.makedirs(self.root, exist_ok=True)
+        for name, a in self.arrays.items():
+            np.save(os.path.join(self.root, name + ".npy"), a)
+
+
 # =====================================================================================================================
 # CPU legs (the only code in this file that touches oracle/)
 # =====================================================================================================================
@@ -244,7 +275,7 @@ def cpu_sae_tokens_per_sec(budget_s=12.0, threads=None, batch=1024):
 
 
 def run_reference_arm(args):
-    """The reference's own CPU path (its restatement, oracle/: /root/reference does not exist on the GPU box) on this box's host
+    """The reference's own CPU path (its restatement, oracle/) on this box's host
     cores, same metric / unit / workload as the product arm's headline, each step a bounded sample of that workload.  Rank 0 only."""
     world, rank, _ = _dist()
     if rank != 0:
@@ -358,7 +389,7 @@ def time_dominant_gemm(model, batch, dtype, iters=10):
     return {"ms": ms, "flops": 2.0 * M * N * K, "bytes": float(M * K * es + N * K * es + 2 * M * N * es), "shape": [M, N, K]}
 
 
-def run_vit(args, ctx, cpu_leg=True):
+def run_vit(args, ctx, cpu_leg=True, dump=None):
     from vit_prisma.b200 import _lib as L
     from vit_prisma.b200.synthetic import CLIP_B32, CLIP_L14
     world, rank, dev = ctx.world, ctx.rank, ctx.dev
@@ -385,16 +416,23 @@ def run_vit(args, ctx, cpu_leg=True):
     with clocks:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(args.steps):
+        for i in range(args.steps):
             out, cache = model.run_with_cache(x, **run_kw)
             n_keys = len(cache)
-            del cache
+            if dump is None or i < args.steps - 1:
+                del cache
         e1.record()
         ctx.barrier()
         dev_ms = ctx.max_over_ranks(e0.elapsed_time(e1))
     clocks.close()
     launches = L.get_lib().pb_launch_count() - launches0
     route = model.last_route
+    if dump is not None:
+        rec_name = f"vit_{args.model}_{args.dtype}"
+        dump.add(f"{rec_name}.out", out)
+        for name, t in cache.items():                      # 214 hook points at B/32: a small sample of each
+            dump.add(f"{rec_name}.cache.{name}", t, cap=1 << 14)
+        del cache
 
     # ---- end to end: pinned host batch -> H2D -> run_with_cache -> D2H of the model output, every step
     # result read back every step: the model output [B, n_classes]; with stop_at_layer the output is the residual stream
@@ -528,7 +566,16 @@ def build_sae_trainer(ctx, cfg, store, group=None, init=None):
     return trainer
 
 
-def run_sae(args, ctx, spec=None):
+def dump_train_step(dump, rec_name, out, sae):
+    """VisionSAETrainer.train_step's return values and the parameters the step left in the module."""
+    names = ("loss", "mse_loss", "l1_loss", "l0", "act_freq_scores", "n_forward_passes_since_fired", "n_frac_active_tokens")
+    for name, value in zip(names, out):
+        dump.add(f"{rec_name}.{name}", value)
+    for name, t in sae.state_dict().items():
+        dump.add(f"{rec_name}.{name}", t)
+
+
+def run_sae(args, ctx, spec=None, dump=None):
     """``spec`` = SAE_CFG (the headline, configs[2]) or SAE_CFG5 (configs[4]: bf16 storage -- parameters, state dict and activations
     in bf16; the step engine trains fp32 masters and exports the rounded parameters every step, vit_prisma/sae/sae.py)."""
     from vit_prisma.b200 import _lib as L
@@ -563,6 +610,7 @@ def run_sae(args, ctx, spec=None):
         state["step"] += 1
         state["tokens"] += Bt * world
         state["n_frac"] = out[-1]
+        state["out"] = out
         return out[0]                                     # loss: 0-dim device tensor
 
     clocks = ClockSampler(ctx.local, period_s=0.002)
@@ -582,6 +630,8 @@ def run_sae(args, ctx, spec=None):
         dev_ms = ctx.max_over_ranks(e0.elapsed_time(e1))
     clocks.close()
     launches = L.get_lib().pb_launch_count() - l0
+    if dump is not None:
+        dump_train_step(dump, "sae_train" if spec is SAE_CFG else "sae_train_cfg5", state["out"], sae)
     assert sae.step_engine() is eng, "the step engine was rebuilt during training"
 
     # ---- e2e: pinned host tokens -> H2D -> VisionSAETrainer.train_step -> D2H of the step's loss
@@ -664,7 +714,7 @@ def run_sae(args, ctx, spec=None):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-def run_sae_forward(args, ctx, expansion=64):
+def run_sae_forward(args, ctx, expansion=64, dump=None):
     """north_star's forward-only shape: SAE encoder -> TopK -> decoder at d_model 768, dict 768 x 64, 4096 tokens per call,
     against SURVEY 8(d)'s forward bytes `4*(2*Bt*d) + 4*d*F + 4*F + 4*d*min(F, Bt*k)` (sparse outputs; no dense feature_acts).
     Every rank runs its own replica (no collective); the record reports the sum."""
@@ -677,7 +727,7 @@ def run_sae_forward(args, ctx, expansion=64):
     unit_norm_rows_(eng.W_dec)
     eng.refresh_lo()
     pool = activation_pool(Bt * 8, d, seed=ctx.rank).to(ctx.dev)
-    n = max(args.steps, 10)
+    n = args.steps
     # warm-up by time, not by count: on rank 0 this record follows ~12 s of host-only work (the CPU baseline) during which the GPU
     # idles and drops its clocks; a handful of 0.7 ms calls is not enough to bring them back before the timed region starts
     t_warm, i = time.perf_counter(), 0
@@ -692,10 +742,13 @@ def run_sae_forward(args, ctx, expansion=64):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(n):
-        eng.forward(pool[(i % 8) * Bt:(i % 8 + 1) * Bt])
+        res = eng.forward(pool[(i % 8) * Bt:(i % 8 + 1) * Bt])
     e1.record()
     ctx.barrier()
     ms = ctx.max_over_ranks(e0.elapsed_time(e1)) / n
+    if dump is not None:
+        for name, t in zip(("sae_out", "idx", "val"), res):
+            dump.add(f"sae_forward.{name}", t)
     fb_rows, rescored = eng.fallback_rows(), eng.rescored_per_row(Bt)
 
     def phase_ms(bits, reps=5):                       # one phase of the fused encode alone, warm replays
@@ -736,7 +789,7 @@ def run_sae_forward(args, ctx, expansion=64):
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-def run_cfg4(args, ctx):
+def run_cfg4(args, ctx, dump=None):
     """BASELINE.json configs[3]: CLIP ViT-L/14 run_with_cache feeding an SAE (d_model 1024, dict 1024 x 64, TopK 32), data parallel:
     every rank runs its own VisionActivationsStore over its own synthetic image shard (names_filter = one resid_post,
     stop_at_layer = layer + 1, exactly the store's call) and trains on its own token shard through VisionSAETrainer.train_step;
@@ -776,6 +829,7 @@ def run_cfg4(args, ctx):
                                  n_training_steps=state["step"], n_training_tokens=state["step"] * Bt * world)
         state["step"] += 1
         state["n_frac"] = out[-1]
+        state["out"] = out
         return out[0]
 
     for _ in range(args.warmup):
@@ -788,6 +842,8 @@ def run_cfg4(args, ctx):
     e1.record()
     ctx.barrier()
     ms = ctx.max_over_ranks(e0.elapsed_time(e1))
+    if dump is not None:
+        dump_train_step(dump, "cfg4_sae_train", state["out"], sae)
     if rank != 0:
         return None
     tokens = world * Bt * args.steps
@@ -807,13 +863,14 @@ def run_cfg4(args, ctx):
 def dp_parity_gate(ctx):
     """N > 1 only, after the timed regions: the NVLink data-parallel step, driven through VisionSAETrainer(p2p_group=...), must
     reproduce the reference's single-process training of tests/golden/sae_tiny_b.pt (fixture made by the unmodified reference):
-    global mse, grad norm, bit-exact TopK indices, parameters after steps 0 / 2 / 5, dead-feature counters, and identical
+    global mse, grad norm, bit-exact TopK indices, parameters after steps 0 / 5, dead-feature counters, and identical
     parameters on every rank.  Returns (ok, detail) on every rank."""
     import torch.distributed as dist
     from vit_prisma.b200.p2p import P2PGroup, SaeDPEngine
     from vit_prisma.sae.train_sae import FusedAdamHandle, FusedSchedule
     from vit_prisma.sae.training.get_scheduler import lr_multiplier_fn
-    gold = torch.load(os.path.join(ROOT, "tests", "golden", "sae_tiny_b.pt"), weights_only=False)
+    from tests.util import load_golden
+    gold = load_golden("sae_tiny_b.pt")
     world, rank, dev = ctx.world, ctx.rank, ctx.dev
     B, d, k, F = gold["batch"], gold["d_in"], gold["k"], gold["d_sae"]
     g = torch.Generator().manual_seed(gold["data_seed"])
@@ -896,31 +953,34 @@ def main():
     ap.add_argument("--batch", type=int, default=512, help="ViT images per step per GPU")
     ap.add_argument("--model", default="b32", choices=["b32", "l14"], help="l14 = cfg #4: ViT-L/14 with the activation store's names_filter / stop_at_layer")
     ap.add_argument("--layer", type=int, default=22, help="hook_resid_post layer cached by --model l14")
-    ap.add_argument("--vit-steps", type=int, default=None, help="steps of the secondary ViT record under --workload all (default: min(steps, 10))")
+    ap.add_argument("--vit-steps", type=int, default=None, help="steps of the secondary ViT records under --workload all (default: --steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what each timed path returned in its last timed step to DIR/*.npy (at most 64 MB, see OutputDump)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference_arm(args)
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device -- the product path has no CPU fallback (use --impl reference for the CPU arm)")
     ctx = Ctx()
+    dump = OutputDump(args.dump_outputs) if args.dump_outputs and ctx.rank == 0 else None
     rc = 0
     try:
         line = None
         if args.workload == "cfg4":
-            line = run_cfg4(args, ctx)
+            line = run_cfg4(args, ctx, dump=dump)
         if args.workload == "cfg5":
-            line = run_sae(args, ctx, spec=SAE_CFG5)
+            line = run_sae(args, ctx, spec=SAE_CFG5, dump=dump)
         if args.workload == "sae_fwd":
-            line = run_sae_forward(args, ctx)
+            line = run_sae_forward(args, ctx, dump=dump)
         if args.workload in ("all", "sae"):
-            line = run_sae(args, ctx)
+            line = run_sae(args, ctx, dump=dump)
             if ctx.world > 1:
                 ok, detail = dp_parity_gate(ctx)
                 if line is not None:
                     line["dp_parity"], line["dp_parity_detail"] = ok, detail
                 rc = 0 if ok else 3
             try:                                           # north_star's forward-only shape (dict 768 x 64), nested; never costs the headline
-                fwd = run_sae_forward(args, ctx)
+                fwd = run_sae_forward(args, ctx, dump=dump)
             except Exception as e:                         # noqa: BLE001 -- reported in the line, not swallowed
                 fwd = {"error": f"{type(e).__name__}: {e}"}
             if line is not None and fwd is not None:
@@ -928,19 +988,21 @@ def main():
         if args.workload in ("all", "vit"):
             vargs = argparse.Namespace(**vars(args))
             if args.workload == "all":
-                vargs.steps = args.vit_steps or min(args.steps, 10)
+                vargs.steps = args.vit_steps or args.steps
                 vargs.warmup = min(args.warmup, 3)
-            vit = run_vit(vargs, ctx)
+            vit = run_vit(vargs, ctx, dump=dump)
             if args.workload == "vit":
                 line = vit
             elif line is not None:
                 line["secondary"] = vit
             if args.workload == "all" and args.dtype == "fp32":      # the throughput mode of the same path: bf16 operands, fp32 accumulation
                 vargs.dtype = "bf16"
-                vit16 = run_vit(vargs, ctx, cpu_leg=False)
+                vit16 = run_vit(vargs, ctx, cpu_leg=False, dump=dump)
                 if line is not None and vit16 is not None:
                     vit16["cpu_baseline"] = vit["cpu_baseline"] if vit else None
                     line["secondary_bf16"] = vit16
+        if dump is not None:
+            dump.write()
         if ctx.rank == 0 and line is not None:
             print(json.dumps(line), flush=True)
     finally:

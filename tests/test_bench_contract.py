@@ -40,6 +40,35 @@ def test_reference_arm_nonzero_ranks_exit_quietly():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_output_dump_samples_the_same_positions_and_stays_under_budget(tmp_path):
+    """--dump-outputs: float32 for floating point (bf16 included), float64 for integers, large arrays sampled at positions that do
+    not change from run to run, and a refusal instead of writing more than OutputDump.BUDGET."""
+    import numpy as np
+    from bench import OutputDump
+    g = torch.Generator().manual_seed(1)
+    x, n = torch.randn(3_000_000, generator=g), torch.arange(12, dtype=torch.int32).reshape(3, 4)
+    for run in ("a", "b"):
+        dump = OutputDump(str(tmp_path / run))
+        dump.add("big", x)
+        dump.add("small", x[:10].bfloat16())
+        dump.add("idx", n)
+        dump.add("absent", None)
+        dump.write()
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["big.npy", "idx.npy", "small.npy"] and files == sorted(os.listdir(tmp_path / "b"))
+    big, idx, small = (np.load(tmp_path / "a" / f) for f in files)
+    assert big.dtype == np.float32 and big.shape == (1 << 20,) and np.array_equal(big, np.load(tmp_path / "b" / "big.npy"))
+    assert np.isin(big, x.numpy()).all()
+    assert idx.dtype == np.float64 and np.array_equal(idx, n.numpy())
+    assert small.dtype == np.float32 and small.shape == (10,)
+    dump = OutputDump(str(tmp_path / "c"))
+    for i in range(17):
+        dump.add(f"a{i}", x)
+    with pytest.raises(SystemExit):
+        dump.write()
+    assert not (tmp_path / "c").exists()
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU refusal")
 def test_product_arm_fails_loudly_without_a_gpu():
     out = _run("--steps", "1", "--warmup", "1")

@@ -162,13 +162,31 @@ def test_conditional_hook_gates_on_cpu():
     m.reset_hooks()
 
 
+_REFUSAL = """
+import pytest, torch
+from vit_prisma.b200._lib import PrismaB200Error
+from vit_prisma.configs.HookedViTConfig import HookedViTConfig
+from vit_prisma.models.base_vit import HookedViT
+assert not torch.cuda.is_available()
+m = HookedViT(HookedViTConfig(1, 8, 8, 8))
+with pytest.raises(PrismaB200Error, match="no CPU fallback"):
+    m(torch.rand(1, 3, 224, 224))
+with pytest.raises(PrismaB200Error):
+    m.run_with_cache(torch.rand(1, 3, 224, 224))
+print("refused")
+"""
+
+
 def test_product_path_refuses_cpu_tensors():
-    from vit_prisma.b200._lib import PrismaB200Error
-    m = HookedViT(HookedViTConfig(1, 8, 8, 8))
-    with pytest.raises(PrismaB200Error, match="no CPU fallback"):
-        m(torch.rand(1, 3, 224, 224))
-    with pytest.raises(PrismaB200Error):
-        m.run_with_cache(torch.rand(1, 3, 224, 224))
+    """With no CUDA device visible, a call on host tensors raises instead of computing on the host.  (With one, a host-resident
+    model is staged on the GPU instead, DESIGN.md section 1.)  Run in a child process that sees no device, so that the refusal is
+    checked on machines with a GPU too."""
+    import subprocess
+    import sys
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    env["PYTHONPATH"] = os.pathsep.join([os.path.join(ROOT, "vit-prisma_b200"), env.get("PYTHONPATH", "")])
+    out = subprocess.run([sys.executable, "-c", _REFUSAL], env=env, cwd=ROOT, capture_output=True, text=True, timeout=300)
+    assert out.returncode == 0 and out.stdout.strip().endswith("refused"), (out.stdout + out.stderr)[-3000:]
 
 
 def test_c_abi_library_exports_every_declared_symbol():

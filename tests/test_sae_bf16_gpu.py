@@ -97,7 +97,6 @@ def test_bf16_sae_trains_on_fp32_masters_and_exports_bf16_parameters():
     assert torch.equal(eng2.W_dec.cpu(), gold["init"]["W_dec"].float())
 
 
-@pytest.mark.skip(reason="written after the round's GPU minutes were spent: never run on hardware, so it cannot vouch for anything yet")
 def test_bf16_module_routes_agree_and_hooks_see_bf16():
     """A bf16 module computes in fp32 on its masters on BOTH routes: the sparse engine route (no hooks) and the module-by-module route
     (a HookPoint is live).  Hooks see tensors rounded to cfg.dtype -- the reference's rounding points -- and the two routes agree to

@@ -1,4 +1,6 @@
 """Parity helpers shared by the tests (SURVEY section 7 step 1)."""
+import io
+import lzma
 import os
 
 import torch
@@ -7,7 +9,12 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def load_golden(name):
-    return torch.load(os.path.join(GOLDEN, name), weights_only=False)
+    """tests/golden/<name>, or its LZMA-compressed form <name>.xz (golden/compact_golden.py)."""
+    path = os.path.join(GOLDEN, name)
+    if os.path.exists(path):
+        return torch.load(path, weights_only=False)
+    with open(path + ".xz", "rb") as f:
+        return torch.load(io.BytesIO(lzma.decompress(f.read())), weights_only=False)
 
 
 def rel_err(got: torch.Tensor, ref: torch.Tensor) -> float:
