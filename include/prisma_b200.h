@@ -233,15 +233,19 @@ typedef struct {
   /* scratch of pb_sae_backward for features selected by more than 64 tokens (their lists are split across warps):
    * work_bytes >= 8 + 4*F + 8*(rows*k/32 + F + 1)                                                                        */
   void* work; int64_t work_bytes;
-  /* [2] max_f ||W_encT[f,:]||_2 and max_f ||W_encT[f,:] - tf32_trunc(.)||_2 AFTER this step's update, for the fused encoder's error bound
+  /* [2] max_f ||W_encT[f,:]||_2 and max_f ||W_encT[f,:] - f16(.)||_2 AFTER this step's update, for the fused encoder's error bound
    * (pb_sae_encode_topk_fused); may be NULL                                                                               */
   float* enc_norm_max;
   /* 1: pb_sae_step_reset already zeroed gcol / gbdec2 / the work header for this step (pb_sae_backward then skips its memsets) */
   int32_t pre_zeroed;
+  /* fp16 [F][(d + 7) & ~7] shadow of W_encT for the fused encoder's candidate GEMM, rewritten by pb_sae_adam; may be NULL.
+   * f16(x): round to nearest, saturate to +-65504, results below 2^-14 in magnitude flushed to zero                         */
+  void* W_encT_h;
 } PbSaeStep;
 
-/* sae_in = norm_in(x) - b_dec (+ tf32 residual, row mean / std, column sums of x) -- sae.py:78-87, 557-566 */
-PB_API int pb_sae_prep(const float* x, const float* b_dec, float* sae_in, float* sae_in_lo, float* mu, float* sd,
+/* sae_in = norm_in(x) - b_dec (+ tf32 residual, fp16 shadow [rows][(d + 7) & ~7] for the fused encoder, row mean / std, column
+ * sums of x) -- sae.py:78-87, 557-566; sae_in_lo, sae_in_h, xsum may be NULL                                                */
+PB_API int pb_sae_prep(const float* x, const float* b_dec, float* sae_in, float* sae_in_lo, void* sae_in_h, float* mu, float* sd,
                        float* xsum, int32_t rows, int32_t d, int32_t norm_mode, pb_stream_t stream);
 /* torch.topk(hidden_pre, k, dim=-1) (sae.py:803-805): idx int32 / val fp32 [rows][k], sorted by value descending,
  * ties broken towards the lower index; feat_count[f] += 1 per selection (may be NULL);
@@ -268,11 +272,12 @@ PB_API int pb_unit_norm_rows(float* W, float* W_lo, int32_t F, int32_t d, pb_str
 
 /* ------------------------------------------------ fused encoder -> TopK (no dense hidden_pre in HBM)
  * Replaces `hidden_pre = sae_in @ W_enc + b_enc` (sae/sae.py:568-574) + `torch.topk(hidden_pre, k)` (TopK.forward, :803-805) by
- *   phase 1  one-pass TF32 tcgen05 GEMM whose epilogue keeps, per token and per 128-feature segment, the c_keep largest
+ *   phase 1  one-pass fp16 tcgen05 GEMM (kind::f16, fp32 accumulate) on the shadows sae_in_h / W_encT_h, whose epilogue keeps, per token and per 128-feature segment, the c_keep largest
  *            values as packed keys (cand: int32 [rows][d_sae / 128][c_keep]);
  *   phase 2  per token: the m_cand best keys (16 more per round, up to 128, while the proof below fails), EXACT fp32
  *            re-evaluation of those pre-activations, exact top-k of them, and a completeness proof with the per-row bound
- *            |tf32 product - exact| <= ||a - trunc(a)|| max_f||w_f|| + ||a|| max_f||w_f - trunc(w_f)||; rows that fail are listed;
+ *            |fp16 product - exact| <= ||a - f16(a)|| max_f||w_f|| + ||a|| max_f||w_f - f16(w_f)|| + d 2^-22 ||a|| max_f||w_f||
+ *            (operand rounding + fp32 accumulation); rows that fail are listed;
  *   phase 4  exact recomputation + selection for the listed rows (normally none).
  * Same outputs and ordering rules as pb_sae_topk.  phases = 0 runs all three.                                             */
 typedef struct {
@@ -284,18 +289,21 @@ typedef struct {
   const float* sae_in;          /* [rows][d]                                                                              */
   const float* W_encT;          /* [F][d] feature-major encoder                                                           */
   const float* b_enc;           /* [F]                                                                                    */
-  const float* enc_norm_max;    /* [2] max_f ||W_encT[f,:]||, max_f ||W_encT[f,:] - tf32_trunc(.)|| (pb_rownorm_max / pb_sae_adam) */
+  const float* enc_norm_max;    /* [2] max_f ||W_encT[f,:]||, max_f ||W_encT[f,:] - f16(.)|| (pb_rownorm_max / pb_sae_adam) */
   int32_t* cand; int64_t cand_bytes;
   int32_t* idx; float* val;     /* [rows][k]                                                                              */
   float* feat_count;            /* [F] += selections, may be NULL                                                         */
   int32_t* fb_count;            /* [2]: rows that took the exact path in this call; candidates re-scored over the other rows */
   int32_t* fb_rows;             /* [rows]                                                                                 */
   float* fb_scratch; int64_t fb_scratch_bytes;   /* >= F * 4 bytes; one d_sae row per resident CTA of the exact path      */
+  const void* sae_in_h;         /* fp16 [rows][(d + 7) & ~7] = f16(sae_in)  (pb_sae_prep)                                  */
+  const void* W_encT_h;         /* fp16 [F][(d + 7) & ~7]    = f16(W_encT)  (pb_rownorm_max / pb_sae_adam)                 */
 } PbSaeEncode;
 PB_API int pb_sae_fused_workspace(int32_t rows, int32_t F, int32_t c_keep, int64_t* cand_bytes, int64_t* fb_scratch_bytes);
 PB_API int pb_sae_encode_topk_fused(const PbSaeEncode* e, pb_stream_t stream);
-/* out[0] = max_f ||W[f,:]||_2, out[1] = max_f ||W[f,:] - tf32_trunc(W[f,:])||_2 over the rows of a contiguous fp32 [F][d] matrix */
-PB_API int pb_rownorm_max(const float* W, int32_t F, int32_t d, float* out, pb_stream_t stream);
+/* out[0] = max_f ||W[f,:]||_2, out[1] = max_f ||W[f,:] - f16(W[f,:])||_2 over the rows of a contiguous fp32 [F][d] matrix, and
+ * (W_h != NULL) the fp16 shadow W_h [F][(d + 7) & ~7] = f16(W): one pass rebuilds everything the fused encoder derives from W */
+PB_API int pb_rownorm_max(const float* W, int32_t F, int32_t d, float* out, void* W_h, pb_stream_t stream);
 
 /* ------------------------------------------------ dense SAE step pieces (activation_fn_str = "relu" + L1) and ghost grads
  * StandardSparseAutoencoder.forward with a dense activation executes six [tokens x d_sae x d_in] products
@@ -392,9 +400,6 @@ PB_API int pb_p2p_barrier(const PbP2PStep* s, uint32_t epoch, pb_stream_t stream
 PB_API int pb_p2p_sum_xsum(const PbP2PStep* s, float* xsum_global, pb_stream_t stream);
 PB_API int pb_p2p_reduce_scatter(const PbP2PStep* s, pb_stream_t stream);
 PB_API int pb_p2p_adam_allgather(const PbP2PStep* s, pb_stream_t stream);
-/* after the barrier that follows pb_p2p_adam_allgather: enc_norm_max[0..1] (PbSaeEncode.enc_norm_max) = max over ranks of the
- * encoder row-norm maxima each rank measured on its owned rows; norm_parts must hold 3 * PB_P2P_MAX_RANKS floats, part_accum 4 */
-PB_API int pb_p2p_wmax(const PbP2PStep* s, float* enc_norm_max, pb_stream_t stream);
 PB_API int pb_p2p_push_dec(const PbP2PStep* s, pb_stream_t stream);        /* the deferred W_dec half of the all-gather (defer_dec = 1) */
 /* NVSwitch multicast memory (csrc/mc.cu).  Collective protocol, driven from the host side (vit_prisma/b200/p2p.py):
  *   every rank pb_mc_supported -> rank 0 pb_mc_create (fd) -> fd to the other ranks (SCM_RIGHTS) -> pb_mc_import ->

@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
@@ -95,6 +96,26 @@ __device__ __forceinline__ float tf32_lo(float x) {
   uint32_t r;
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x - tf32_trunc(x)));
   return __uint_as_float(r);
+}
+
+// fp16 operand of the fused encoder's candidate GEMM (sae_in_h, W_encT_h): round to nearest, saturate to +-65504, and flush
+// results below 2^-14 in magnitude to zero.  Every producer of the fp16 shadows and every residual norm of the error bound uses
+// this one conversion.  The flush makes the software residual x - f16_val(h) exact whatever the tensor core does with fp16
+// subnormals; saturation turns an overflow into a huge residual, so the bound fails and the row takes the exact path.
+__device__ __forceinline__ uint16_t f16_cand(float x) {
+  uint16_t h;
+  asm("cvt.rn.satfinite.f16.f32 %0, %1;" : "=h"(h) : "f"(x));
+  return (h & 0x7c00u) == 0 ? (uint16_t)0 : h;
+}
+__device__ __forceinline__ float f16_val(uint16_t h) { return __half2float(__ushort_as_half(h)); }
+// row stride (elements) of the fp16 shadows: rows padded to 16 bytes, as the tensor maps require
+__host__ __device__ __forceinline__ int f16_ld(int d) { return (d + 7) & ~7; }
+// four consecutive fp16 operands (8 bytes) + the sum of squares of their residuals
+__device__ __forceinline__ float st4_f16_cand(uint16_t* p, const float v[4]) {
+  const uint16_t h0 = f16_cand(v[0]), h1 = f16_cand(v[1]), h2 = f16_cand(v[2]), h3 = f16_cand(v[3]);
+  if (p) *reinterpret_cast<uint2*>(p) = make_uint2((uint32_t)h0 | ((uint32_t)h1 << 16), (uint32_t)h2 | ((uint32_t)h3 << 16));
+  const float r0 = v[0] - f16_val(h0), r1 = v[1] - f16_val(h1), r2 = v[2] - f16_val(h2), r3 = v[3] - f16_val(h3);
+  return r0 * r0 + r1 * r1 + r2 * r2 + r3 * r3;
 }
 
 // ------------------------------------------------------------- activations

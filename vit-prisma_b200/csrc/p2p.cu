@@ -119,7 +119,7 @@ __global__ void k_p2p_sum_small(P2PTables t, float* __restrict__ out, int which,
 // four dependent ~4 us launches in front of the reduce-scatter); thread 0 also resets the step's accumulators
 __global__ void __launch_bounds__(256) k_p2p_sum_small3(P2PTables t, float* __restrict__ gb_enc_red, float* __restrict__ gb_dec_red,
                                                        float* __restrict__ fired_red, int F, int d, float* __restrict__ part_accum) {
-  if (blockIdx.x == 0 && threadIdx.x < 4) part_accum[threadIdx.x] = 0.f;   // [0] gradient-norm partial, [1..2] encoder row-norm maxima of the owned slice
+  if (blockIdx.x == 0 && threadIdx.x < 4) part_accum[threadIdx.x] = 0.f;   // [0] gradient-norm partial of the owned slice
   const int n = 2 * F + d;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const int which = i < F ? 0 : i < 2 * F ? 1 : 2;
@@ -263,10 +263,8 @@ __global__ void __launch_bounds__(256) k_p2p_adam_allgather(P2PTables t, int f0,
                                                            float* __restrict__ m_dec, float* __restrict__ v_dec, float* __restrict__ m_enc,
                                                            float* __restrict__ v_enc, float* __restrict__ m_be, float* __restrict__ v_be,
                                                            const SaeScalarsP2P* __restrict__ sc, AdamHyperP2P h, float* __restrict__ mc_W_dec,
-                                                           float* __restrict__ mc_W_encT, float* __restrict__ mc_b_enc, float* __restrict__ wmax_accum,
-                                                           int defer_dec) {
+                                                           float* __restrict__ mc_W_encT, float* __restrict__ mc_b_enc, int defer_dec) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  float enc_best = 0.f, enc_best_lo = 0.f;
   const int nvec = d >> 2;
   const float clip = sc->clip_coef;
   float* W_dec = t.W_dec[t.rank];
@@ -326,7 +324,6 @@ __global__ void __launch_bounds__(256) k_p2p_adam_allgather(P2PTables t, int f0,
         else for (int j = 0; j < t.world; ++j) st4(wdec_rot[j] + base + 4 * c4, w[i]);     // all-gather: peer stores, own copy first
       }
     }
-    float esq = 0.f, elo = 0.f;
 #pragma unroll
     for (int i = 0; i < CHUNKS; ++i) {
       const int c4 = i * 32 + lane;
@@ -340,9 +337,6 @@ __global__ void __launch_bounds__(256) k_p2p_adam_allgather(P2PTables t, int f0,
         for (int q = 0; q < 4; ++q) {
           p[q] = adam_upd(p[q], gr[q] * clip, mm[q], vv[q], h);
           lo[q] = tf32_lo(p[q]);
-          esq = fmaf(p[q], p[q], esq);
-          const float tl = p[q] - tf32_trunc(p[q]);
-          elo = fmaf(tl, tl, elo);
         }
         st4(m_enc + base + 4 * c4, mm);
         st4(v_enc + base + 4 * c4, vv);
@@ -356,8 +350,6 @@ __global__ void __launch_bounds__(256) k_p2p_adam_allgather(P2PTables t, int f0,
         }
       }
     }
-    enc_best = fmaxf(enc_best, warp_sum(esq));
-    enc_best_lo = fmaxf(enc_best_lo, warp_sum(elo));
     if (lane == 0) {
       float mm = m_be[f], vv = v_be[f];
       const float nb = adam_upd(t.b_enc[t.rank][f], gb_enc_red[f] * clip, mm, vv, h);
@@ -367,34 +359,14 @@ __global__ void __launch_bounds__(256) k_p2p_adam_allgather(P2PTables t, int f0,
       else for (int r = 0; r < t.world; ++r) t.b_enc[r][f] = nb;
     }
   }
-  // largest encoder-column norms of the OWNED rows (error bound of the fused encoder's tf32 pass); merged across ranks by pb_p2p_wmax
-  if (wmax_accum && lane == 0 && enc_best > 0.f) {
-    atomicMax(reinterpret_cast<unsigned int*>(wmax_accum), __float_as_uint(sqrtf(enc_best)));
-    atomicMax(reinterpret_cast<unsigned int*>(wmax_accum) + 1, __float_as_uint(sqrtf(enc_best_lo)));
-  }
-}
-
-// norm_parts layout on every rank: [0, 8) gradient-norm partials, [8, 16) max ||w_f|| partials, [16, 24) max ||w_f - trunc(w_f)|| partials
-__global__ void k_p2p_wmax_reduce(P2PTables t, float* __restrict__ enc_norm_max) {
-  float a = 0.f, b = 0.f;
-  for (int r = 0; r < t.world; ++r) {
-    a = fmaxf(a, t.norm_parts[t.rank][PB_MAX_RANKS + r]);
-    b = fmaxf(b, t.norm_parts[t.rank][2 * PB_MAX_RANKS + r]);
-  }
-  enc_norm_max[0] = a;
-  enc_norm_max[1] = b;
 }
 
 // replicated tiny updates: b_dec Adam (identical inputs on every rank -> identical result) and the dead-feature counters
-__global__ void __launch_bounds__(256) k_p2p_small_updates(P2PTables t, const float* __restrict__ wmax_accum, float* __restrict__ b_dec,
+__global__ void __launch_bounds__(256) k_p2p_small_updates(P2PTables t, float* __restrict__ b_dec,
                                                           const float* __restrict__ gb_dec_red, float* __restrict__ m_bd,
                                                           float* __restrict__ v_bd, const float* __restrict__ fired_red,
                                                           float* __restrict__ since_fired, float* __restrict__ act_freq,
                                                           const SaeScalarsP2P* __restrict__ sc, AdamHyperP2P h, int d, int F) {
-  if (blockIdx.x == 0 && threadIdx.x < t.world) {      // publish this rank's encoder row-norm maxima to every peer (was its own launch)
-    t.norm_parts[threadIdx.x][PB_MAX_RANKS + t.rank] = wmax_accum[0];
-    t.norm_parts[threadIdx.x][2 * PB_MAX_RANKS + t.rank] = wmax_accum[1];
-  }
   const float clip = sc->clip_coef;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < F; i += gridDim.x * blockDim.x) {
     if (i < d) {
@@ -480,7 +452,7 @@ extern "C" int pb_p2p_adam_allgather(const PbP2PStep* s, pb_stream_t stream) {
   int grid = pb_sm_count() * 4;
   if (grid > (per + 7) / 8) grid = (per + 7) / 8;
   PB_CHECK_ARG((!s->mc_W_dec == !s->mc_W_encT) && (!s->mc_W_dec == !s->mc_b_enc), "pb_p2p_adam_allgather: all three multicast parameter views or none");
-#define PB_P2P_ADAM(CH) k_p2p_adam_allgather<CH><<<grid, 256, 0, st>>>(t, f0, f1, d, s->gb_enc_red, s->m_dec, s->v_dec, s->m_enc, s->v_enc, s->m_be, s->v_be, (const SaeScalarsP2P*)s->scalars, h, s->mc_W_dec, s->mc_W_encT, s->mc_b_enc, s->part_accum + 1, s->defer_dec)
+#define PB_P2P_ADAM(CH) k_p2p_adam_allgather<CH><<<grid, 256, 0, st>>>(t, f0, f1, d, s->gb_enc_red, s->m_dec, s->v_dec, s->m_enc, s->v_enc, s->m_be, s->v_be, (const SaeScalarsP2P*)s->scalars, h, s->mc_W_dec, s->mc_W_encT, s->mc_b_enc, s->defer_dec)
   const int nvec = d / 4;
   if (d % 4 != 0 || nvec > 384) { pb_set_error("pb_p2p_adam_allgather: d_in=%d unsupported", d); return PB_EUNSUPPORTED; }
   if (nvec <= 32) PB_P2P_ADAM(1);
@@ -491,7 +463,7 @@ extern "C" int pb_p2p_adam_allgather(const PbP2PStep* s, pb_stream_t stream) {
   else PB_P2P_ADAM(12);
 #undef PB_P2P_ADAM
   PB_LAUNCH_CHECK();
-  k_p2p_small_updates<<<(s->F + 255) / 256, 256, 0, st>>>(t, s->part_accum + 1, s->b_dec, s->gb_dec_red, s->m_bd, s->v_bd, s->fired_red, s->since_fired,
+  k_p2p_small_updates<<<(s->F + 255) / 256, 256, 0, st>>>(t, s->b_dec, s->gb_dec_red, s->m_bd, s->v_bd, s->fired_red, s->since_fired,
                                                         s->act_freq, (const SaeScalarsP2P*)s->scalars, h, d, s->F);
   PB_LAUNCH_CHECK();
   return PB_OK;
@@ -519,16 +491,6 @@ extern "C" int pb_p2p_push_dec(const PbP2PStep* s, pb_stream_t stream) {
   PB_TRY(fill_tables(s, &t));
   const int per = s->F / s->world, f0 = s->rank * per, f1 = f0 + per;
   k_p2p_push_dec<<<pb_sm_count() * 2, 256, 0, (cudaStream_t)stream>>>(t, f0, f1, s->d, s->mc_W_dec);
-  PB_LAUNCH_CHECK();
-  return PB_OK;
-}
-
-// after the barrier that follows pb_p2p_adam_allgather: enc_norm_max[0..1] = max over ranks of the published row-norm maxima
-extern "C" int pb_p2p_wmax(const PbP2PStep* s, float* enc_norm_max, pb_stream_t stream) {
-  P2PTables t;
-  PB_TRY(fill_tables(s, &t));
-  PB_CHECK_ARG(enc_norm_max, "pb_p2p_wmax: output missing");
-  k_p2p_wmax_reduce<<<1, 1, 0, (cudaStream_t)stream>>>(t, enc_norm_max);
   PB_LAUNCH_CHECK();
   return PB_OK;
 }

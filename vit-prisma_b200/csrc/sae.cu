@@ -33,13 +33,14 @@ struct SaeScalars {
 // ---------------------------------------------------------------------------------------------
 // 1. prep: run-time input normalisation + decoder-bias subtraction (sae.py:78-87, 557-566)
 //    layer_norm mode: mu = mean(x); xc = x - mu; std = unbiased std(xc); xn = xc / (std + 1e-5)
-//    sae_in = xn - b_dec ;  sae_in_lo = tf32 residual (A operand of the 3xTF32 encoder GEMM)
+//    sae_in = xn - b_dec ;  sae_in_lo = tf32 residual (A operand of the 3xTF32 encoder GEMM) ;
+//    sae_in_h = f16_cand(sae_in), row stride f16_ld(d) (A operand of the fused encoder's candidate GEMM)
 //    xsum[c] += x[b,c]  (batch mean for _compute_mse_loss's centring, sae.py:145)
 // one warp per token row; row kept in registers.
 template <int CHUNKS>
 __global__ void __launch_bounds__(256) k_sae_prep(const float* __restrict__ x, const float* __restrict__ b_dec, float* __restrict__ sae_in,
-                                                  float* __restrict__ sae_in_lo, float* __restrict__ mu_out, float* __restrict__ std_out,
-                                                  int rows, int d, int norm_mode, float eps) {
+                                                  float* __restrict__ sae_in_lo, uint16_t* __restrict__ sae_in_h, float* __restrict__ mu_out,
+                                                  float* __restrict__ std_out, int rows, int d, int norm_mode, float eps) {
   pb_pdl();
   const int lane = threadIdx.x & 31;
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -95,6 +96,7 @@ __global__ void __launch_bounds__(256) k_sae_prep(const float* __restrict__ x, c
       (void)inv;
       st4(sae_in + (int64_t)row * d + 4 * c4, o);
       if (sae_in_lo) st4(sae_in_lo + (int64_t)row * d + 4 * c4, lo);
+      if (sae_in_h) st4_f16_cand(sae_in_h + (int64_t)row * f16_ld(d) + 4 * c4, o);
     }
   }
 }
@@ -745,7 +747,8 @@ __global__ void __launch_bounds__(256) k_sae_adam_rows(float* __restrict__ W_dec
                                                        float* __restrict__ v_enc, float* __restrict__ m_be, float* __restrict__ v_be,
                                                        const float* __restrict__ fired, float* __restrict__ since_fired,
                                                        float* __restrict__ act_freq, const SaeScalars* __restrict__ sc, AdamHyper h,
-                                                       int F, int d, int renorm, float* __restrict__ enc_norm_max) {
+                                                       int F, int d, int renorm, float* __restrict__ enc_norm_max,
+                                                       uint16_t* __restrict__ W_encT_h) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
   const int nvec = d >> 2;
   const float clip = sc->clip_coef;
@@ -814,9 +817,8 @@ __global__ void __launch_bounds__(256) k_sae_adam_rows(float* __restrict__ W_dec
           p[q] = adam_update(p[q], gr[q] * clip, mm[q], vv[q], h);
           lo[q] = tf32_lo(p[q]);
           esq = fmaf(p[q], p[q], esq);
-          const float tl = p[q] - tf32_trunc(p[q]);
-          elo = fmaf(tl, tl, elo);
         }
+        elo += st4_f16_cand(W_encT_h ? W_encT_h + (int64_t)f * f16_ld(d) + 4 * c4 : nullptr, p);
         st4(W_encT + base + 4 * c4, p);
         st4(m_enc + base + 4 * c4, mm);
         st4(v_enc + base + 4 * c4, vv);
@@ -834,7 +836,7 @@ __global__ void __launch_bounds__(256) k_sae_adam_rows(float* __restrict__ W_dec
       if (act_freq) act_freq[f] += fired[f];
     }
   }
-  // largest encoder-column norm after the update (error bound of the fused encoder's tf32 pass); norms are >= 0 so the
+  // largest encoder-column norm after the update (error bound of the fused encoder's fp16 pass); norms are >= 0 so the
   // bit pattern orders like the value
   if (enc_norm_max && lane == 0 && enc_best > 0.f) {
     atomicMax(reinterpret_cast<unsigned int*>(enc_norm_max), __float_as_uint(sqrtf(enc_best)));
@@ -870,7 +872,8 @@ k_sae_adam_bulk(float* __restrict__ W_dec, float* __restrict__ W_encT, float* __
                 float* __restrict__ m_enc, float* __restrict__ v_enc, float* __restrict__ m_be, float* __restrict__ v_be,
                 const float* __restrict__ fired, float* __restrict__ since_fired, float* __restrict__ act_freq,
                 const SaeScalars* __restrict__ sc, AdamHyper h, int F, int d, int renorm, float* __restrict__ enc_norm_max, int S,
-                float* __restrict__ b_dec, const float* __restrict__ gb_dec, float* __restrict__ m_bd, float* __restrict__ v_bd) {
+                float* __restrict__ b_dec, const float* __restrict__ gb_dec, float* __restrict__ m_bd, float* __restrict__ v_bd,
+                uint16_t* __restrict__ W_encT_h) {
   pb_pdl_trigger();
   extern __shared__ __align__(128) unsigned char ab_smem[];
   const uint32_t s0 = smem_u32(ab_smem);
@@ -996,9 +999,8 @@ k_sae_adam_bulk(float* __restrict__ W_dec, float* __restrict__ W_encT, float* __
         for (int q = 0; q < 4; ++q) {
           p[q] = adam_update(p[q], gr[q] * clip, mm[q], vv[q], h);
           esq = fmaf(p[q], p[q], esq);
-          const float tl = p[q] - tf32_trunc(p[q]);
-          elo = fmaf(tl, tl, elo);
         }
+        elo += st4_f16_cand(W_encT_h ? W_encT_h + (int64_t)f * f16_ld(d) + 4 * c4 : nullptr, p);   // fp16 shadow: from registers
         st4(we + 4 * c4, p);
         st4(me + 4 * c4, mm);
         st4(ve + 4 * c4, vv);
@@ -1110,14 +1112,15 @@ static int persistent_grid(int warps_per_cta, int items) {
   return ctas < 1 ? 1 : ctas;
 }
 
-extern "C" int pb_sae_prep(const float* x, const float* b_dec, float* sae_in, float* sae_in_lo, float* mu, float* sd, float* xsum, int32_t rows,
-                           int32_t d, int32_t norm_mode, pb_stream_t stream) {
+extern "C" int pb_sae_prep(const float* x, const float* b_dec, float* sae_in, float* sae_in_lo, void* sae_in_h, float* mu, float* sd, float* xsum,
+                           int32_t rows, int32_t d, int32_t norm_mode, pb_stream_t stream) {
   PB_CHECK_ARG(x && b_dec && sae_in && rows >= 0 && d > 0, "pb_sae_prep: bad arguments");
   PB_CHECK_ARG(norm_mode == 0 || (mu && sd), "pb_sae_prep: mu/std buffers required when normalising");
   if (rows == 0) return PB_OK;
   cudaStream_t st = (cudaStream_t)stream;
   const int ch = chunks_for(d);
-  PB_DISPATCH_CHUNKS(ch, PB_LAUNCH_PDL(k_sae_prep<C_>, (rows + 7) / 8, 256, 0, st, x, b_dec, sae_in, sae_in_lo, mu, sd, rows, d, norm_mode, 1e-5f));
+  PB_DISPATCH_CHUNKS(ch, PB_LAUNCH_PDL(k_sae_prep<C_>, (rows + 7) / 8, 256, 0, st, x, b_dec, sae_in, sae_in_lo, reinterpret_cast<uint16_t*>(sae_in_h), mu, sd, rows,
+                                          d, norm_mode, 1e-5f));
   if (xsum) {
     PB_CUDA(cudaMemsetAsync(xsum, 0, sizeof(float) * d, st));
     const int rpc = 8;
@@ -1308,7 +1311,8 @@ extern "C" int pb_sae_adam(const PbSaeStep* s, pb_stream_t stream) {
     PB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                                     \
     PB_LAUNCH_PDL(kern, g2, 32 * (1 + S), smem, st, s->W_dec, s->W_encT, s->b_enc, s->gW_dec, s->gW_encT, s->gb_enc, s->m_dec, s->v_dec, s->m_enc, \
                   s->v_enc, s->m_be, s->v_be, s->fired, s->since_fired, s->act_freq, (const SaeScalars*)s->scalars,                    \
-                  h, F, d, s->renorm_decoder, s->enc_norm_max, S, s->b_dec, s->gb_dec, s->m_bd, s->v_bd);                               \
+                  h, F, d, s->renorm_decoder, s->enc_norm_max, S, s->b_dec, s->gb_dec, s->m_bd, s->v_bd,                                \
+                  reinterpret_cast<uint16_t*>(s->W_encT_h));                                                                          \
   } while (0)
       switch (ch) {
         case 1: PB_ADAM_BULK(1); break;
@@ -1326,7 +1330,8 @@ extern "C" int pb_sae_adam(const PbSaeStep* s, pb_stream_t stream) {
   PB_DISPATCH_CHUNKS(ch, (k_sae_adam_rows<C_><<<grid, 256, 0, st>>>(s->W_dec, s->W_encT, s->W_encT_lo, s->b_enc, s->gW_dec, s->gW_encT, s->gb_enc,
                                                                      s->m_dec, s->v_dec, s->m_enc, s->v_enc, s->m_be, s->v_be, s->fired,
                                                                      s->since_fired, s->act_freq, (const SaeScalars*)s->scalars, h,
-                                                                     F, d, s->renorm_decoder, s->enc_norm_max)));
+                                                                     F, d, s->renorm_decoder, s->enc_norm_max,
+                                                                     reinterpret_cast<uint16_t*>(s->W_encT_h))));
   PB_LAUNCH_CHECK();
   k_sae_adam_vec<<<(d + 255) / 256, 256, 0, st>>>(s->b_dec, s->gb_dec, s->m_bd, s->v_bd, (const SaeScalars*)s->scalars, h, d);
   PB_LAUNCH_CHECK();

@@ -2,11 +2,11 @@
 // written to HBM (reference sae/sae.py:557-581 `sae_in @ W_enc + b_enc` followed by TopK.forward :795-808 `torch.topk`).
 //
 // Approximate-then-rescore, exact by construction:
-//   1. k_enc_cand     persistent tcgen05 GEMM, ONE kind::tf32 pass (the fp32 operands are read by the tensor core with their 13
-//                     low mantissa bits ignored), 128 x 256 tiles, accumulators double-buffered in TMEM.  The epilogue never
-//                     stores the tile: every thread owns one token row x 128 feature columns of it (TMEM's native layout) and
-//                     keeps that segment's C_KEEP largest values as packed keys (order-preserving int of the value, the low
-//                     7 bits replaced by the column inside the segment) with a branch-free insertion network, then writes
+//   1. k_enc_cand     persistent tcgen05 GEMM, ONE kind::f16 pass over the fp16 shadows sae_in_h / W_encT_h (f16_cand: round to
+//                     nearest, saturate, flush below 2^-14; fp32 accumulate), 128 x 256 tiles, accumulators double-buffered in
+//                     TMEM.  The epilogue never stores the tile: every thread owns one token row x 128 feature columns of it
+//                     (TMEM's native layout) and keeps that segment's C_KEEP largest values as packed keys (order-preserving
+//                     int of the value, the low 7 bits replaced by the column inside the segment) with branch-free networks, then writes
 //                     C_KEEP x 4 bytes.  Per token: d_sae / 128 segments x C_KEEP keys (6 KB at d_sae = 24576) instead of a
 //                     98 KB dense row.
 //   2. k_cand_select  one CTA per token: the m_cand best keys of the row (threshold from per-thread bests, rank by counting),
@@ -14,8 +14,8 @@
 //                     exact top-k of the re-scored values (ties -> lower index, sorted descending), and a proof that no
 //                     feature outside the candidate set can belong to the exact top-k:
 //                         ub(best key not selected, or last kept key of a segment whose keys were all selected) + E_row < tau_k
-//                     where E_row bounds |tf32 product - exact| by Cauchy-Schwarz: 2^-9 ||sae_in_row|| max_f ||W_enc[:, f]||
-//                     (each operand loses < 2^-10 relative to truncation).  Rows that fail the proof go on a list.
+//                     where E_row bounds |fp16 product - exact| by Cauchy-Schwarz on the operand residuals plus the fp32
+//                     accumulation (DESIGN.md section 4).  Rows that fail the proof go on a list.
 //   3. k_topk_fallback  persistent, normally finds the list empty: recomputes a listed row's 'd_sae' pre-activations exactly and
 //                     selects from all of them.  Correctness therefore never depends on the approximation; only speed does.
 // Outputs are those of pb_sae_topk: idx int32 / val fp32 [rows][k] sorted by value, feat_count[f] += selections.
@@ -40,20 +40,51 @@ constexpr int FZ_STAGES = 4;     // 4 x (16 KB A + 32 KB B) = 192 KB operand rin
 constexpr int FZ_NEPI = 8;       // epilogue warps: 4 TMEM lane quarters x 2 column halves
 constexpr int FZ_SEG = 128;      // columns per thread segment (= FZ_BN / 2)
 constexpr int FZ_THREADS = 64 + FZ_NEPI * 32;
-using FzCfg = TcCfg<float, 1, FZ_BN, FZ_STAGES>;
+using FzCfg = TcCfg<uint16_t, 1, FZ_BN, FZ_STAGES>;    // fp16 operands: 64 elements per 128-byte k-slab
+// kind::f16 instruction descriptor: c_format F32 [4,6) | a_format = b_format = F16 (0) | K-major | N>>3 [17,23) | M>>4 [24,29)
+constexpr uint32_t FZ_IDESC = (1u << 4) | ((uint32_t)(FZ_BN >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
 constexpr int FZ_SMEM = FzCfg::RING_BYTES + 1024 + 256;
+
+// Insert x into s[0, N) (sorted descending) and drop the smallest of the N + 1: 2N - 1 integer min / max.
+template <int N>
+__device__ __forceinline__ void key_insert(int (&s)[N], int x) {
+#pragma unroll
+  for (int i = 0; i < N - 1; ++i) {
+    const int hi = max(s[i], x);
+    x = min(s[i], x);
+    s[i] = hi;
+  }
+  s[N - 1] = max(s[N - 1], x);
+}
+__device__ __forceinline__ void key_cas(int& a, int& b) {        // a >= b afterwards
+  const int hi = max(a, b);
+  b = min(a, b);
+  a = hi;
+}
 
 // One epilogue warp's share of one finished accumulator: thread = one token row x one 128-feature segment; keeps the segment's
 // C_KEEP largest pre-activations as packed keys and writes them.  `release` is called once the accumulator has been read.
+// Grouped selection: each group of 4 consecutive columns is sorted (5 compare-exchanges) and its r-th largest key goes to a list
+// of floor(C_KEEP / r) slots.  If a group's r-th key is among the segment's C_KEEP largest, so are the r - 1 keys above it, so at
+// most floor(C_KEEP / r) r-th keys are; each list therefore keeps every key of its rank that belongs to the top C_KEEP.  Keys are
+// distinct (the low 7 bits are the column), and the lists are merged once per segment: the same C_KEEP keys, sorted descending,
+// as a plain insertion network, at 9.5 instead of 15 min / max per element for C_KEEP = 8.
 template <int C_KEEP, typename Release>
 __device__ __forceinline__ void enc_cand_epilogue(uint32_t tmem_base, int ab, int quarter, int cbase, int lane, int m0, int n0, int M, int N,
                                                   const float* __restrict__ bias, int* __restrict__ cand, Release release) {
+  constexpr int N2 = C_KEEP / 2, N3 = C_KEEP / 3, N4 = C_KEEP / 4;
   const int nseg = N / FZ_SEG;
   const int row = m0 + quarter * 32 + lane;
   const bool seg_in = (n0 + cbase) < N;          // N % 128 == 0: a segment is entirely inside or outside the matrix
-  int s[C_KEEP];
+  int s[C_KEEP], s2[N2], s3[N3], s4[N4];
 #pragma unroll
   for (int i = 0; i < C_KEEP; ++i) s[i] = INT_MIN;
+#pragma unroll
+  for (int i = 0; i < N2; ++i) s2[i] = INT_MIN;
+#pragma unroll
+  for (int i = 0; i < N3; ++i) s3[i] = INT_MIN;
+#pragma unroll
+  for (int i = 0; i < N4; ++i) s4[i] = INT_MIN;
 #pragma unroll 1
   for (int c = 0; c < FZ_SEG / 32; ++c) {
     uint32_t r[32];
@@ -70,20 +101,24 @@ __device__ __forceinline__ void enc_cand_epilogue(uint32_t tmem_base, int ab, in
       for (int q = 0; q < 8; ++q) {
         float bb[4];
         ld4(bp + 4 * q, bb);                     // same address in every lane: one broadcast transaction
+        int x[4];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          int x = (f2ord(__uint_as_float(r[4 * q + j]) + bb[j]) & ~127) | (c * 32 + 4 * q + j);
-#pragma unroll
-          for (int i = 0; i < C_KEEP; ++i) {     // insertion network: s[] stays sorted descending
-            const int hi = max(s[i], x);
-            x = min(s[i], x);
-            s[i] = hi;
-          }
-        }
+        for (int j = 0; j < 4; ++j) x[j] = (f2ord(__uint_as_float(r[4 * q + j]) + bb[j]) & ~127) | (c * 32 + 4 * q + j);
+        key_cas(x[0], x[1]); key_cas(x[2], x[3]); key_cas(x[0], x[2]); key_cas(x[1], x[3]); key_cas(x[1], x[2]);
+        key_insert(s, x[0]);
+        key_insert(s2, x[1]);
+        key_insert(s3, x[2]);
+        key_insert(s4, x[3]);
       }
     }
   }
   if (seg_in && row < M) {
+#pragma unroll
+    for (int i = 0; i < N2; ++i) key_insert(s, s2[i]);
+#pragma unroll
+    for (int i = 0; i < N3; ++i) key_insert(s, s3[i]);
+#pragma unroll
+    for (int i = 0; i < N4; ++i) key_insert(s, s4[i]);
     int* dst = cand + ((int64_t)row * nseg + (n0 + cbase) / FZ_SEG) * C_KEEP;
     if (C_KEEP % 4 == 0) {
 #pragma unroll
@@ -155,7 +190,7 @@ k_enc_cand(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
       }
     }
   } else if (warp == 1) {
-    // ===================== MMA issuer: one kind::tf32 pass =====================
+    // ===================== MMA issuer: one kind::f16 pass =====================
     if (lane == 0) {
       uint32_t it = 0;
       int li = 0;
@@ -175,7 +210,7 @@ k_enc_cand(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
 #pragma unroll
           for (int k = 0; k < 128 / C::UMMA_K_BYTES; ++k) {
             const uint32_t koff = k * C::UMMA_K_BYTES;
-            tc_mma<1>(d_tmem, make_smem_desc(sa + koff), make_smem_desc(sb + koff), C::IDESC, (kb | k) != 0 ? 1u : 0u);
+            tc_mma<0>(d_tmem, make_smem_desc(sa + koff), make_smem_desc(sb + koff), FZ_IDESC, (kb | k) != 0 ? 1u : 0u);
           }
           tc_commit(empty_bar(s));
         }
@@ -214,7 +249,7 @@ k_enc_cand(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
 constexpr int FZP_STAGES = 6;
 constexpr int FZP_A_BYTES = TC_BM * 128, FZP_BH_BYTES = (FZ_BN / 2) * 128, FZP_STAGE_BYTES = FZP_A_BYTES + FZP_BH_BYTES;
 constexpr int FZP_SMEM = FZP_STAGES * FZP_STAGE_BYTES + 1024 + 256;
-constexpr uint32_t FZP_IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(FZ_BN >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);   // tf32, M = 256 across the pair
+constexpr uint32_t FZP_IDESC = (1u << 4) | ((uint32_t)(FZ_BN >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);   // f16, M = 256 across the pair
 
 template <int C_KEEP>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(FZ_THREADS, 1)
@@ -236,7 +271,7 @@ k_enc_cand_pair(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   const uint32_t rank = cluster_ctarank();
   const bool leader = rank == 0;
   const int cluster_id = blockIdx.x >> 1, n_clusters = gridDim.x >> 1;
-  constexpr int BK = 32;
+  constexpr int BK = 64;                                   // fp16 elements per 128-byte k-slab
   const int num_kb = (K + BK - 1) / BK;
   const int num_tiles = num_m_tiles * num_n_tiles;
   auto tile_m = [&](int tile) { return tile % num_m_tiles; };        // m-fastest raster, as in k_enc_cand
@@ -278,7 +313,7 @@ k_enc_cand_pair(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       }
     }
   } else if (warp == 1) {
-    if (leader && lane == 0) {                               // MMA issuer (leader only): one kind::tf32 pass
+    if (leader && lane == 0) {                               // MMA issuer (leader only): one kind::f16 pass
       uint32_t it = 0;
       int li = 0;
       for (int tile = cluster_id; tile < num_tiles; tile += n_clusters, ++li) {
@@ -296,7 +331,7 @@ k_enc_cand_pair(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           const uint32_t sb = sa + FZP_A_BYTES;
 #pragma unroll
           for (int k = 0; k < 4; ++k)
-            tc_mma_pair<1>(d_tmem, make_smem_desc(sa + 32 * k), make_smem_desc(sb + 32 * k), FZP_IDESC, (kb | k) != 0 ? 1u : 0u);
+            tc_mma_pair<0>(d_tmem, make_smem_desc(sa + 32 * k), make_smem_desc(sb + 32 * k), FZP_IDESC, (kb | k) != 0 ? 1u : 0u);
           tc_commit_pair(empty_bar(s));
         }
         tc_commit_pair(tfull_bar(ab));
@@ -387,7 +422,7 @@ __global__ void __launch_bounds__(256) k_cand_select(const int* __restrict__ can
   const int nvec = d >> 2;
   const int nkeys = nseg * c_keep;
 
-  // ---- the token's encoder input -> shared memory; ||a|| and ||a - tf32_trunc(a)|| for the error bound
+  // ---- the token's encoder input -> shared memory; ||a|| and ||a - f16_cand(a)|| for the error bound
   {
     const float4* src = reinterpret_cast<const float4*>(sae_in + (int64_t)row * d);
     float4* dst = reinterpret_cast<float4*>(a_row);
@@ -396,8 +431,8 @@ __global__ void __launch_bounds__(256) k_cand_select(const int* __restrict__ can
       const float4 v = src[i];
       dst[i] = v;
       nsq += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
-      const float lx = v.x - tf32_trunc(v.x), ly = v.y - tf32_trunc(v.y), lz = v.z - tf32_trunc(v.z), lw = v.w - tf32_trunc(v.w);
-      lsq += lx * lx + ly * ly + lz * lz + lw * lw;
+      const float vv[4] = {v.x, v.y, v.z, v.w};
+      lsq += st4_f16_cand(nullptr, vv);
     }
     nsq = warp_sum(nsq);
     lsq = warp_sum(lsq);
@@ -547,8 +582,10 @@ __global__ void __launch_bounds__(256) k_cand_select(const int* __restrict__ can
       const int u_rest = m_cur < G ? sel_key(items[m_cur]) : u_below;                      // best key not re-scored
       const int u = max(u_rest, sat_key);
       const float u_val = u == INT_MIN ? -INFINITY : ord2f((u & ~127) | 127);               // upper end of the key's value bucket
-      // |tf32 product - exact| = |a_lo.w + a_hi.w_lo| <= ||a_lo|| max||w|| + ||a|| max||w_lo||   (Cauchy-Schwarz, per row)
-      const float E = err_scale * (a_lo_norm * wnorm_max[0] + a_norm * wnorm_max[1]) + fabsf(tau_exact) * 1.2207031e-4f;
+      // |fp16 product - exact| <= ||a_lo|| max||w|| + ||a|| max||w_lo|| (operands, Cauchy-Schwarz, per row, lo = x - f16_cand(x))
+      //                          + d 2^-22 ||a|| max||w||                 (fp32 accumulation in the tensor core: DESIGN.md section 4)
+      const float E = err_scale * (a_lo_norm * wnorm_max[0] + a_norm * wnorm_max[1] + (float)d * 2.3841858e-7f * a_norm * wnorm_max[0]) +
+                      fabsf(tau_exact) * 1.2207031e-4f;
       ok = !overflow && m_cur >= k && (u_val + E < tau_exact);
     }
     if (ok || m_cur >= Gs) break;
@@ -638,9 +675,10 @@ __global__ void __launch_bounds__(256) k_topk_fallback(const int* __restrict__ f
   }
 }
 
-// out[0] = max_f ||W[f, :]||_2, out[1] = max_f ||W[f, :] - tf32_trunc(W[f, :])||_2 (atomic max on the bit patterns: norms are
-// non-negative); out must be zeroed by the caller
-__global__ void __launch_bounds__(256) k_rownorm_max(const float* __restrict__ W, int F, int d, float* __restrict__ out) {
+// out[0] = max_f ||W[f, :]||_2, out[1] = max_f ||W[f, :] - f16_cand(W[f, :])||_2 (atomic max on the bit patterns: norms are
+// non-negative), and the fp16 shadow W_h[f, :] = f16_cand(W[f, :]) (row stride f16_ld(d)) when W_h is given; out must be zeroed
+// by the caller
+__global__ void __launch_bounds__(256) k_rownorm_max(const float* __restrict__ W, int F, int d, float* __restrict__ out, uint16_t* __restrict__ W_h) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
   const int nvec = d >> 2;
   float best = 0.f, best_lo = 0.f;
@@ -650,8 +688,8 @@ __global__ void __launch_bounds__(256) k_rownorm_max(const float* __restrict__ W
     for (int i = lane; i < nvec; i += 32) {
       const float4 v = w4[i];
       s += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
-      const float lx = v.x - tf32_trunc(v.x), ly = v.y - tf32_trunc(v.y), lz = v.z - tf32_trunc(v.z), lw = v.w - tf32_trunc(v.w);
-      l += lx * lx + ly * ly + lz * lz + lw * lw;
+      const float vv[4] = {v.x, v.y, v.z, v.w};
+      l += st4_f16_cand(W_h ? W_h + (int64_t)f * f16_ld(d) + 4 * i : nullptr, vv);
     }
     best = fmaxf(best, warp_sum(s));
     best_lo = fmaxf(best_lo, warp_sum(l));
@@ -671,8 +709,8 @@ static int enc_pair_mode() {
 template <int C_KEEP>
 int launch_enc_cand_pair(const PbSaeEncode* e, cudaStream_t st) {
   CUtensorMap tmA, tmBh;
-  PB_TRY(make_map(&tmA, e->sae_in, PB_F32, e->rows, e->d, e->d, TC_BM));
-  PB_TRY(make_map(&tmBh, e->W_encT, PB_F32, e->F, e->d, e->d, FZ_BN / 2));       // box = this CTA's half of the dictionary tile
+  PB_TRY(make_map(&tmA, e->sae_in_h, TC_F16, e->rows, e->d, f16_ld(e->d), TC_BM));
+  PB_TRY(make_map(&tmBh, e->W_encT_h, TC_F16, e->F, e->d, f16_ld(e->d), FZ_BN / 2));       // box = this CTA's half of the dictionary tile
   auto kern = k_enc_cand_pair<C_KEEP>;
   static bool attr_done = false;
   if (!attr_done) {
@@ -691,8 +729,8 @@ int launch_enc_cand(const PbSaeEncode* e, cudaStream_t st) {
   const int pm = enc_pair_mode();
   if (pm == 1 || (pm < 0 && PB_ENC_PAIR_DEFAULT && e->rows >= 512)) return launch_enc_cand_pair<C_KEEP>(e, st);
   CUtensorMap tmA, tmB;
-  PB_TRY(make_map(&tmA, e->sae_in, PB_F32, e->rows, e->d, e->d, TC_BM));
-  PB_TRY(make_map(&tmB, e->W_encT, PB_F32, e->F, e->d, e->d, FZ_BN));
+  PB_TRY(make_map(&tmA, e->sae_in_h, TC_F16, e->rows, e->d, f16_ld(e->d), TC_BM));
+  PB_TRY(make_map(&tmB, e->W_encT_h, TC_F16, e->F, e->d, f16_ld(e->d), FZ_BN));
   auto kern = k_enc_cand<C_KEEP>;
   static bool attr_done = false;
   if (!attr_done) {
@@ -725,14 +763,16 @@ extern "C" int pb_sae_fused_workspace(int32_t rows, int32_t F, int32_t c_keep, i
 }
 
 extern "C" int pb_sae_encode_topk_fused(const PbSaeEncode* e, pb_stream_t stream) {
-  PB_CHECK_ARG(e && e->sae_in && e->W_encT && e->b_enc && e->cand && e->enc_norm_max && e->idx && e->val && e->fb_count && e->fb_rows,
+  PB_CHECK_ARG(e && e->sae_in && e->W_encT && e->sae_in_h && e->W_encT_h && e->b_enc && e->cand && e->enc_norm_max && e->idx && e->val &&
+                   e->fb_count && e->fb_rows,
                "pb_sae_encode_topk_fused: missing pointers");
   PB_CHECK_ARG(e->rows >= 0 && e->d >= 32 && e->d % 4 == 0 && e->d <= 8192 && e->F % FZ_SEG == 0 && e->F >= FZ_SEG,
                "pb_sae_encode_topk_fused: needs d_in %% 4 == 0, 32 <= d_in <= 8192, d_sae %% 128 == 0 (d=%d F=%d)", e->d, e->F);
   PB_CHECK_ARG(e->c_keep == 4 || e->c_keep == 6 || e->c_keep == 8, "pb_sae_encode_topk_fused: c_keep must be 4, 6 or 8");
   PB_CHECK_ARG(e->k >= 1 && e->k <= 64 && e->k <= e->m_cand && e->m_cand <= SEL_MAX_CAND && e->k <= e->F,
                "pb_sae_encode_topk_fused: needs k <= 64 and k <= m_cand <= %d", SEL_MAX_CAND);
-  PB_CHECK_ARG(pb_aligned16(e->sae_in) && pb_aligned16(e->W_encT) && pb_aligned16(e->b_enc) && pb_aligned16(e->cand),
+  PB_CHECK_ARG(pb_aligned16(e->sae_in) && pb_aligned16(e->W_encT) && pb_aligned16(e->sae_in_h) && pb_aligned16(e->W_encT_h) &&
+                   pb_aligned16(e->b_enc) && pb_aligned16(e->cand),
                "pb_sae_encode_topk_fused: operands must be 16-byte aligned");
   const int nkeys = e->F / FZ_SEG * e->c_keep;
   PB_CHECK_ARG(e->F / FZ_SEG <= 256 * 4, "pb_sae_encode_topk_fused: d_sae=%d too large for the selection kernel (max 131072)", e->F);
@@ -772,14 +812,15 @@ extern "C" int pb_sae_encode_topk_fused(const PbSaeEncode* e, pb_stream_t stream
   return PB_OK;
 }
 
-extern "C" int pb_rownorm_max(const float* W, int32_t F, int32_t d, float* out, pb_stream_t stream) {
+extern "C" int pb_rownorm_max(const float* W, int32_t F, int32_t d, float* out, void* W_h, pb_stream_t stream) {
   PB_CHECK_ARG(W && out && F >= 0 && d > 0 && d % 4 == 0, "pb_rownorm_max: bad arguments");
+  PB_CHECK_ARG(pb_aligned16(W_h), "pb_rownorm_max: W_h must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   PB_CUDA(cudaMemsetAsync(out, 0, 2 * sizeof(float), st));
   if (F == 0) return PB_OK;
   int grid = pb_sm_count() * 4;
   if (grid > (F + 7) / 8) grid = (F + 7) / 8;
-  k_rownorm_max<<<grid, 256, 0, st>>>(W, F, d, out);
+  k_rownorm_max<<<grid, 256, 0, st>>>(W, F, d, out, reinterpret_cast<uint16_t*>(W_h));
   PB_LAUNCH_CHECK();
   return PB_OK;
 }

@@ -130,16 +130,18 @@ EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
+constexpr int TC_F16 = 2;   // make_map dtype of the fp16 operands (PB_F32 / PB_BF16 for the others)
+
 // 2-D map over a row-major [rows, cols] matrix with row stride ld (elements); box = [box_rows, 128 bytes]
 int make_map(CUtensorMap* map, const void* ptr, int dtype, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
   EncodeTiledFn fn = get_encode_fn();
   if (!fn) { pb_set_error("gemm_tc: cuTensorMapEncodeTiled entry point unavailable"); return PB_ECUDA; }
-  const int es = dtype == PB_BF16 ? 2 : 4;
+  const int es = dtype == PB_F32 ? 4 : 2;
   cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   cuuint64_t gstride[1] = {(cuuint64_t)ld * es};
   cuuint32_t box[2] = {(cuuint32_t)(128 / es), (cuuint32_t)box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult rc = fn(map, dtype == PB_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(ptr), gdim,
+  CUresult rc = fn(map, dtype == PB_F32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : dtype == PB_BF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(ptr), gdim,
                    gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (rc != CUDA_SUCCESS) {

@@ -46,7 +46,6 @@ L.register_signatures({
     "pb_p2p_sum_xsum": (i32, [C.POINTER(PbP2PStep), vp, vp]),
     "pb_p2p_reduce_scatter": (i32, [C.POINTER(PbP2PStep), vp]),
     "pb_p2p_adam_allgather": (i32, [C.POINTER(PbP2PStep), vp]),
-    "pb_p2p_wmax": (i32, [C.POINTER(PbP2PStep), vp, vp]),
     "pb_p2p_push_dec": (i32, [C.POINTER(PbP2PStep), vp]),
     "pb_mc_supported": (i32, [C.POINTER(i32)]),
     "pb_mc_round_size": (i32, [i32, i64, C.POINTER(i64)]),
@@ -264,7 +263,7 @@ class SaeDPEngine(SaeStepEngine):
         shared["W_encT"].copy_(W_encT)
         shared["W_dec"].copy_(W_dec)
         shared["b_enc"].copy_(b_enc)
-        for name, shape in (("gb_enc", (F,)), ("gb_dec", (d,)), ("fired", (F,)), ("xsum", (d,)), ("norm_parts", (3 * MAX_RANKS,))):
+        for name, shape in (("gb_enc", (F,)), ("gb_dec", (d,)), ("fired", (F,)), ("xsum", (d,)), ("norm_parts", (MAX_RANKS,))):
             g.alloc(name, shape)
         g.alloc("flags", (MAX_RANKS,), dtype=torch.int32)
         g.alloc("flags2", (MAX_RANKS,), dtype=torch.int32)        # barrier of the side stream that finishes the W_dec all-gather
@@ -278,7 +277,7 @@ class SaeDPEngine(SaeStepEngine):
         self.xsum_local = g.local["xsum"]
         dev = W_dec.device
         self.gb_enc_red, self.gb_dec_red, self.fired_red = torch.zeros(F, device=dev), torch.zeros(d, device=dev), torch.zeros(F, device=dev)
-        self.part_accum = torch.zeros(4, device=dev)        # gradient-norm partial + encoder row-norm maxima of the owned slice
+        self.part_accum = torch.zeros(4, device=dev)        # [0]: gradient-norm partial of the owned slice
         import os
         # PRISMA_P2P_OVERLAP=1: the W_dec half of the all-gather runs on a side stream under the next step's prep / encoder GEMM /
         # select (it is first read by the next decode).  OFF by default: measured no gain at 8 ranks and a loss at 2 (run 17's trace:
@@ -416,9 +415,11 @@ class SaeDPEngine(SaeStepEngine):
             self._mark("side: barrier2 done", self._side)
             self._ev_dec = torch.cuda.Event()
             self._ev_dec.record(self._side)
-        if self.encoder == "fused":                     # error bound of the next step's tf32 pass: largest encoder-column norms, merged over ranks
-            L.check(lib.pb_p2p_wmax(C.byref(ps), self.enc_norm_max.data_ptr(), st), "pb_p2p_wmax")
-        self._mark("wmax")
+        if self.encoder == "fused":
+            # the next step's candidate GEMM reads the fp16 shadow and the encoder-row norm maxima: every rank rebuilds both from its
+            # full, freshly all-gathered W_encT (one local pass; the shadow rows are not pushed over NVLink)
+            self.refresh_lo()
+        self._mark("fp16 shadow refresh")
         return self.scalars
 
     # ------------------------------------------------------------------ instrumentation: COLLECTIVE (every rank must call it)

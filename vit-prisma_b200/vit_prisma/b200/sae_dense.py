@@ -237,7 +237,8 @@ class SaeDenseStepEngine(SaeStepEngine):
         dead_idx = None
         if use_ghost_grads:
             dead_idx = torch.nonzero(since_fired > dead_feature_window).flatten().to(torch.int32)
-        L.check(lib.pb_sae_prep(x.data_ptr(), self.b_dec.data_ptr(), self.sae_in.data_ptr(), self.sae_in_lo.data_ptr(), self.mu.data_ptr(),
+        L.check(lib.pb_sae_prep(x.data_ptr(), self.b_dec.data_ptr(), self.sae_in.data_ptr(), self.sae_in_lo.data_ptr(), None,
+                                self.mu.data_ptr(),
                                 self.sd.data_ptr(), self.xsum.data_ptr(), rows, d, self.norm_mode, st), "pb_sae_prep")
         self.scalars.zero_(); self.aux.zero_(); self.fired.zero_()
         self.step_count += 1

@@ -39,7 +39,7 @@ class PbSaeStep(C.Structure):
             "csc_off", "csc_cursor", "csc_entries", "gW_dec", "gW_encT", "gb_enc", "gb_dec", "gcol", "gbdec2",
             "fired", "scalars", "m_dec", "v_dec", "m_enc", "v_enc", "m_be", "v_be", "m_bd", "v_bd",
             "since_fired", "act_freq")]
-        + [("global_rows", i32), ("dist", i32), ("work", vp), ("work_bytes", i64), ("enc_norm_max", vp), ("pre_zeroed", i32)]
+        + [("global_rows", i32), ("dist", i32), ("work", vp), ("work_bytes", i64), ("enc_norm_max", vp), ("pre_zeroed", i32), ("W_encT_h", vp)]
     )
 
 
@@ -49,12 +49,13 @@ class PbSaeEncode(C.Structure):
         [(n, i32) for n in ("rows", "d", "F", "k", "c_keep", "m_cand", "phases")] + [("err_coef", f32)]
         + [(n, vp) for n in ("sae_in", "W_encT", "b_enc", "enc_norm_max", "cand")] + [("cand_bytes", i64)]
         + [(n, vp) for n in ("idx", "val", "feat_count", "fb_count", "fb_rows", "fb_scratch")] + [("fb_scratch_bytes", i64)]
+        + [(n, vp) for n in ("sae_in_h", "W_encT_h")]
     )
 
 
 L.ABI_STRUCTS.append(PbSaeStep)
 L.register_signatures({
-    "pb_sae_prep": (i32, [vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp]),
+    "pb_sae_prep": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp]),
     "pb_sae_topk": (i32, [vp, i32, i32, i32, vp, vp, vp, vp, i64, vp]),
     "pb_sae_scatter_acts": (i32, [vp, vp, vp, i32, i32, i32, i32, vp]),
     "pb_sae_step_reset": (i32, [C.POINTER(PbSaeStep), vp, vp]),
@@ -65,12 +66,17 @@ L.register_signatures({
     "pb_sae_mse": (i32, [vp, vp, vp, vp, i32, i32, vp]),
     "pb_sae_fused_workspace": (i32, [i32, i32, i32, C.POINTER(i64), C.POINTER(i64)]),
     "pb_sae_encode_topk_fused": (i32, [C.POINTER(PbSaeEncode), vp]),
-    "pb_rownorm_max": (i32, [vp, i32, i32, vp, vp]),
+    "pb_rownorm_max": (i32, [vp, i32, i32, vp, vp, vp]),
 })
 
 NORM_MODE = {"none": 0, None: 0, "layer_norm": 1, "constant_norm_rescale": 2}
 SCALAR_NAMES = ("loss_sum", "gnorm_sq", "clip_coef", "mse", "l0", "pos_count", "grad_norm", "reserved")
 TOPK_SEG = 256 * 96
+
+
+def f16_ld(d: int) -> int:
+    """Row stride (elements) of the fp16 operand shadows of the fused encoder: rows padded to 16 bytes."""
+    return (d + 7) & ~7
 
 
 def unit_norm_rows_(w: torch.Tensor, w_lo: Optional[torch.Tensor] = None) -> None:
@@ -88,7 +94,7 @@ def sae_prep(x2: torch.Tensor, b_dec: torch.Tensor, norm_mode: str):
     sae_in = torch.empty_like(x2)
     mu = torch.empty(rows, device=x2.device)
     sd = torch.empty(rows, device=x2.device)
-    L.check(L.get_lib().pb_sae_prep(x2.data_ptr(), b_dec.data_ptr(), sae_in.data_ptr(), None, mu.data_ptr(), sd.data_ptr(), None,
+    L.check(L.get_lib().pb_sae_prep(x2.data_ptr(), b_dec.data_ptr(), sae_in.data_ptr(), None, None, mu.data_ptr(), sd.data_ptr(), None,
                                     rows, d, NORM_MODE[norm_mode], _stream()), "pb_sae_prep")
     return sae_in, mu, sd
 
@@ -150,7 +156,7 @@ class SaeStepEngine:
         self.gemm_impl = gemm_impl
         dev = W_dec.device
         z = lambda *s, dt=torch.float32: torch.zeros(*s, dtype=dt, device=dev)  # noqa: E731
-        # encoder route: "fused" = one-pass tf32 GEMM with a candidate epilogue + exact re-scoring (csrc/sae_fused.cu, no dense
+        # encoder route: "fused" = one-pass fp16 GEMM with a candidate epilogue + exact re-scoring (csrc/sae_fused.cu, no dense
         # hidden_pre); "dense" = fp32-grade GEMM -> hidden_pre -> k_topk.  "auto" picks fused whenever the geometry allows it and
         # the caller did not pin a GEMM implementation.
         fused_ok = self.d % 4 == 0 and self.d >= 32 and self.F % 128 == 0 and self.k <= 48 and self.F <= 131072
@@ -161,9 +167,11 @@ class SaeStepEngine:
         import os
         self.encoder, self.c_keep = encoder, int(os.environ.get("PRISMA_SAE_C_KEEP", c_keep))     # env overrides: tuning runs only
         self.m_cand = int(os.environ.get("PRISMA_SAE_M_CAND", 0)) or (int(m_cand) if m_cand else self.k + 8)   # first round; +16 per round while unproven
-        self.enc_norm_max = z(2)                      # max ||w_f||, max ||w_f - tf32_trunc(w_f)|| (error bound of the fused encoder)
+        self.enc_norm_max = z(2)                      # max ||w_f||, max ||w_f - f16(w_f)|| (error bound of the fused encoder)
         self.fb_count = z(2, dt=torch.int32)          # rows on the exact path, candidates re-scored (last fused encode)
         self.W_encT_lo = torch.empty_like(W_encT) if encoder == "dense" else None
+        # fp16 shadow of W_encT read by the fused encoder's candidate GEMM; rewritten by every Adam step and by refresh_lo()
+        self.W_encT_h = z(self.F, f16_ld(self.d), dt=torch.float16) if encoder == "fused" else None
         self.refresh_lo()
         # optimizer state (torch.optim.Adam: exp_avg / exp_avg_sq start at zero)
         self.m_dec, self.v_dec, self.m_enc, self.v_enc = z(self.F, self.d), z(self.F, self.d), z(self.F, self.d), z(self.F, self.d)
@@ -180,11 +188,12 @@ class SaeStepEngine:
 
     def refresh_lo(self) -> None:
         """Recompute what the encoder kernels derive from W_enc (after an external write to the parameters): the tf32 residual
-        plane of the dense 3xTF32 route, the largest encoder-column norm of the fused route's error bound."""
+        plane of the dense 3xTF32 route; the fused route's fp16 shadow and the encoder-row norm maxima of its error bound."""
         if self.W_encT_lo is not None:
             from . import ops
             self.W_encT_lo.copy_(ops.split_tf32(self.W_encT))
-        L.check(L.get_lib().pb_rownorm_max(self.W_encT.data_ptr(), self.F, self.d, self.enc_norm_max.data_ptr(), _stream()), "pb_rownorm_max")
+        L.check(L.get_lib().pb_rownorm_max(self.W_encT.data_ptr(), self.F, self.d, self.enc_norm_max.data_ptr(),
+                                           None if self.W_encT_h is None else self.W_encT_h.data_ptr(), _stream()), "pb_rownorm_max")
 
     def _ensure_rows(self, rows: int) -> None:
         if rows == self._rows:
@@ -199,9 +208,11 @@ class SaeStepEngine:
             self.cand = e(max(cb.value // 4, 4), dt=torch.int32)
             self.fb_rows = e(max(rows, 1), dt=torch.int32)
             self.fb_scratch = e(min(64, max(sb.value // (4 * F), 1)) * F)      # exact path: one d_sae row per resident CTA
+            self.sae_in_h = torch.zeros(rows, f16_ld(d), dtype=torch.float16, device=dev)
             self.sae_in_lo = self.hidden_pre = None
         else:
             self.sae_in_lo, self.hidden_pre = e(rows, d), e(rows, F)
+            self.sae_in_h = None
         self.idx, self.val, self.dval = e(rows, k, dt=torch.int32), e(rows, k), e(rows, k)
         self.csc_entries = e(rows * k, dt=torch.int32)
         self.work = e(8 + 4 * F + 8 * (rows * k // 32 + F + 1) + 64, dt=torch.uint8)   # hot-feature work lists (pb_sae_backward)
@@ -228,6 +239,7 @@ class SaeStepEngine:
         s.since_fired, s.act_freq = p(since_fired), p(act_freq)
         s.work, s.work_bytes = p(self.work), self.work.numel()
         s.enc_norm_max = p(self.enc_norm_max)
+        s.W_encT_h = p(self.W_encT_h)
         return s
 
     def _enc_desc(self, rows: int, phases: int = 0) -> PbSaeEncode:
@@ -238,6 +250,7 @@ class SaeStepEngine:
         e.idx, e.val, e.feat_count = self.idx.data_ptr(), self.val.data_ptr(), self.feat_count.data_ptr()
         e.fb_count, e.fb_rows = self.fb_count.data_ptr(), self.fb_rows.data_ptr()
         e.fb_scratch, e.fb_scratch_bytes = self.fb_scratch.data_ptr(), self.fb_scratch.numel() * 4
+        e.sae_in_h, e.W_encT_h = self.sae_in_h.data_ptr(), self.W_encT_h.data_ptr()
         return e
 
     # ------------------------------------------------------------------ pieces
@@ -261,7 +274,7 @@ class SaeStepEngine:
         self._ensure_rows(rows)
         L.check(lib.pb_sae_prep(x.data_ptr(), self.b_dec.data_ptr(), self.sae_in.data_ptr(),
                                 self.sae_in_lo.data_ptr() if (self.sae_in_lo is not None and self.gemm_impl != L.GEMM_SIMT) else None,
-                                self.mu.data_ptr(), self.sd.data_ptr(),
+                                None if self.sae_in_h is None else self.sae_in_h.data_ptr(), self.mu.data_ptr(), self.sd.data_ptr(),
                                 self.xsum.data_ptr(), rows, self.d, self.norm_mode, st), "pb_sae_prep")
         if not pre_zeroed:
             self.feat_count.zero_()
@@ -306,7 +319,7 @@ class SaeStepEngine:
     # ------------------------------------------------------------------ instrumentation (bench.py / tools)
     def describe_encoder(self) -> str:
         if self.encoder == "fused":
-            return (f"fused: one-pass tf32 tcgen05 GEMM with top-{self.c_keep}-per-128-features epilogue -> exact fp32 re-scoring of "
+            return (f"fused: one-pass fp16 tcgen05 GEMM (kind::f16) with top-{self.c_keep}-per-128-features epilogue -> exact fp32 re-scoring of "
                     f">= {self.m_cand} candidates per token -> exact top-{self.k} with a completeness proof (no dense hidden_pre)")
         return "tcgen05 3xTF32 GEMM -> dense hidden_pre -> exact k_topk" if self.gemm_impl != L.GEMM_SIMT else "exact FFMA GEMM -> k_topk"
 
@@ -370,11 +383,11 @@ class SaeStepEngine:
             self.encode_topk(x)
             flops = 2.0 * rows * self.d * self.F
             nkeys = (self.F // 128) * self.c_keep
-            return [("encode + topk, fused (prep + tf32 candidate GEMM + select / exact re-score + exact path)", lambda: self.encode_topk(x),
+            return [("encode + topk, fused (prep + fp16 candidate GEMM + select / exact re-score + exact path)", lambda: self.encode_topk(x),
                      dict(flops=flops, passes=1)),
-                    ("candidate GEMM alone (one tf32 pass, top-c-per-segment epilogue)",
+                    ("candidate GEMM alone (one fp16 pass, top-c-per-segment epilogue)",
                      lambda: L.check(lib.pb_sae_encode_topk_fused(C.byref(self._enc_desc(rows, 1)), st)),
-                     dict(flops=flops, passes=1, bytes=4 * self.d * self.F + 4 * rows * self.d + 4 * rows * nkeys, ncu=r"k_enc_cand")),
+                     dict(flops=flops, passes=1, bytes=2 * self.d * self.F + 2 * rows * self.d + 4 * rows * nkeys, ncu=r"k_enc_cand")),
                     ("select + exact re-score alone", lambda: L.check(lib.pb_sae_encode_topk_fused(C.byref(self._enc_desc(rows, 2)), st)),
                      dict(bytes=4 * rows * nkeys + 4 * rows * self.d + 8 * rows * self.k, ncu=r"k_cand_select"))]
         return [("encode + topk (prep + encoder GEMM 3xTF32 + exact topk)", lambda: self.encode_topk(x),

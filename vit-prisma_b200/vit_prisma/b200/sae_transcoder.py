@@ -57,7 +57,8 @@ class SaeTranscoderStepEngine(SaeDenseStepEngine):
         lib, st = L.get_lib(), _stream()
         rows, d, F = x.shape[0], self.d, self.F
         self._ensure_rows(rows)
-        L.check(lib.pb_sae_prep(x.data_ptr(), self.b_dec.data_ptr(), self.sae_in.data_ptr(), self.sae_in_lo.data_ptr(), self.mu.data_ptr(),
+        L.check(lib.pb_sae_prep(x.data_ptr(), self.b_dec.data_ptr(), self.sae_in.data_ptr(), self.sae_in_lo.data_ptr(), None,
+                                self.mu.data_ptr(),
                                 self.sd.data_ptr(), self.xsum.data_ptr(), rows, d, self.norm_mode, st), "pb_sae_prep")
         self.scalars.zero_(); self.aux.zero_(); self.fired.zero_()
         if self.activation == "relu":
